@@ -5,6 +5,7 @@
          bench.py --gpus N --steps K --warmup W            # one rank per GPU, NCCL
   python bench.py --impl reference ...                     # the reference algorithm on the host CPU cores
   python bench.py --config {posenet,trajcontrol,pipeline,respaced100,lbs}   # the other BASELINE configs (one line each)
+  python bench.py ... --dump-outputs DIR                   # also write the last timed step's outputs as DIR/<name>.npy
 
 Workloads (BASELINE.json configs, per GPU; clips shard over ranks, weak scaling, one all-gather of final outputs per step):
   posenet      configs[1]  PoseNet denoiser, 32 clips x 145 frames (T = 144 motion frames, 145 tokens), 1000 DDPM steps
@@ -35,6 +36,9 @@ import torch
 C_FEATS = 294
 DIFFUSION_STEPS = 1000
 LBS_BYTES_PER_FRAME = 126280  # SURVEY.md 8(d): 10 475 x 3 fp32 vertices + 55 joints out, 145 fp32 in
+DUMP_WHOLE_MAX_ELEMS = 8 << 20  # --dump-outputs: arrays up to 32 MB are written whole, larger ones as a sample
+DUMP_SAMPLE_ELEMS = 1 << 20
+DUMP_LIMIT_BYTES = 64 << 20
 
 CONFIGS = {
     "posenet": dict(clips=32, frames=144, label="BASELINE configs[1]: PoseNet denoiser, batch 32 x 145-frame clips (T=144 "
@@ -379,6 +383,7 @@ class Workload:
         traj = {k[5:]: v.clone() for k, v in batch.items() if k.startswith("traj_")}
         vp, vt, tn = pipeline.run_rounds(self.pargs, self.model, self.tmodel, self.cmodel, self.diff, self.tdiff, self.cdiff,
                                          self.ds_pose, self.ds_traj, self.body, pose, traj)
+        self._traj_out, self._traj_noisy = vt, tn
         self._recon = pipeline.reconstruct_outputs(self.pargs, self.ds_pose, self.body, pose, vp, tn, return_verts=True)
         return vp
 
@@ -403,8 +408,41 @@ class Workload:
     def run(self, batch):
         return getattr(self, "_run_" + self.args.config)(batch)
 
+    def outputs(self, out):
+        """Every array a caller of run() receives from the step that returned `out`, by name."""
+        c = self.args.config
+        if c == "respaced100":
+            return {"pose": out, "traj": self._traj_out}
+        if c == "pipeline":
+            return {"val_output_pose": out, "val_output_traj": self._traj_out, "traj_noisy_full": self._traj_noisy,
+                    **{k: v for k, v in self._recon.items() if v is not None}}
+        if c == "lbs":
+            return {"joints": self._joints, "vertices": out}
+        return {"pose" if c == "posenet" else "traj": out}
+
     def h2d_bytes(self):
         return int(sum(v.numel() * v.element_size() for v in self.host_in.values()))
+
+
+def dump_outputs(dirname, arrays):
+    """Writes each array as <dirname>/<name>.npy (float64 stays float64, everything else becomes float32).  An array of more
+    than DUMP_WHOLE_MAX_ELEMS elements is written as <name>_sample.npy instead: DUMP_SAMPLE_ELEMS elements of its flattened
+    contents at sorted indices drawn from a fixed seed, so two runs with the same shapes sample the same positions."""
+    host = {}
+    for name, t in arrays.items():
+        t = t.detach()
+        if t.dtype != torch.float64:
+            t = t.float()
+        if t.numel() > DUMP_WHOLE_MAX_ELEMS:
+            idx = torch.randint(t.numel(), (DUMP_SAMPLE_ELEMS,), generator=torch.Generator().manual_seed(0)).sort().values
+            t, name = t.reshape(-1)[idx.to(t.device)], name + "_sample"
+        host[name] = t.cpu().numpy()
+    total = sum(a.nbytes for a in host.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise SystemExit(f"--dump-outputs: {total} bytes exceed the {DUMP_LIMIT_BYTES}-byte limit")
+    os.makedirs(dirname, exist_ok=True)
+    for name, a in host.items():
+        np.save(os.path.join(dirname, name + ".npy"), a)
 
 
 def main():
@@ -417,7 +455,11 @@ def main():
     ap.add_argument("--traj-steps", type=int, default=100, help="TrajNet diffusion steps of the pipeline config "
                     "(100 = every shipped RoHM config; 1000 = BASELINE's wording)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last one computed as "
+                    "DIR/<name>.npy (rank 0's clips; arrays over 32 MB as a fixed, seeded sample; 64 MB at most)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         run_reference_arm(args)
         return
@@ -449,10 +491,13 @@ def main():
             dist.barrier()
         torch.cuda.synchronize()
 
+    last = {}
+
     def one_step_resident():
         out = w.run(w.dev_in)
         if gathered is not None:
             dist.all_gather_into_tensor(gathered, out)
+        last["out"] = out
         return out
 
     def one_step_e2e():
@@ -490,6 +535,8 @@ def main():
         barrier()
     ms_per_step = maxreduce(ms_total) / args.steps
     value = world * B / (ms_per_step / 1000.0)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, w.outputs(last["out"]))
 
     one_step_e2e()
     barrier()

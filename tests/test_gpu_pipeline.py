@@ -47,7 +47,7 @@ def _diffusions(dev, traj_steps, pose_steps=1000, pose_respacing=POSE_RESPACING)
 def test_full_pipeline_replays_reference_golden(cuda_device):
     dev = cuda_device
     g = golden("pipeline.npz")
-    B, tn, pn, rounds, s_in, s_pose, s_traj = [int(v) for v in g["meta"]]
+    B, tn, pn, rounds, s_in, s_pose, s_traj, T = [int(v) for v in g["meta"]]
     ds_pose = synthetic.make_dataset('pose', seed=3, realistic_std=True)
     ds_traj = synthetic.make_dataset('traj', seed=3, realistic_std=True)
     mp, mt, mc, *_ = _models(dev, ds_pose, ds_traj)
@@ -57,7 +57,7 @@ def test_full_pipeline_replays_reference_golden(cuda_device):
     dp._randn, dp._randn_like = tape_p.randn, tape_p.randn_like
     for d in (dt, dc):  # the reference's two TrajNet diffusion objects share one module-level RNG stream
         d._randn, d._randn_like = tape_t.randn, tape_t.randn_like
-    pose, traj = synthetic.pipeline_batches(B, s_in, ds_pose, device=dev)
+    pose, traj = synthetic.pipeline_batches(B, s_in, ds_pose, frames=T, device=dev)
     args = pipeline.make_args(sample_iter=rounds, mask_scheme='lower')
     seen = []
 
@@ -70,14 +70,14 @@ def test_full_pipeline_replays_reference_golden(cuda_device):
 
     out_pose, out_traj, traj_noisy = pipeline.run_rounds(args, mp, mt, mc, dp, dt, dc, ds_pose, ds_traj, body, pose, traj,
                                                          on_round=on_round)
-    assert out_pose.shape == (B, 294, 1, 143) and out_traj.shape == (B, 144, 13) and traj_noisy.shape == (B, 144, 22)
+    assert out_pose.shape == (B, 294, 1, T - 1) and out_traj.shape == (B, T, 13) and traj_noisy.shape == (B, T, 22)
     from rohm_b200 import glue
     for it in range(rounds):
         err = {k: float((seen[it][k] - torch.from_numpy(g[f"r{it}_{k}"])).abs().max()) for k in seen[it]}
         # the glue stage on the reference's own TrajNet output (stage-wise): 1e-4.  Free-running, the TrajNet difference
         # (~1e-5) is amplified by the representation itself: velocity channels are frame differences divided by a small Std.
         _, tf_full = glue.traj_to_full_repr(body, torch.from_numpy(g[f"r{it}_val_traj"]).to(dev),
-                                            synthetic.pipeline_batches(B, s_in, ds_pose, device=dev)[1]['motion_repr_clean'],
+                                            synthetic.pipeline_batches(B, s_in, ds_pose, frames=T, device=dev)[1]['motion_repr_clean'],
                                             ds_traj, ds_pose)
         err["traj_full_stagewise"] = float((tf_full.cpu() - torch.from_numpy(g[f"r{it}_traj_full"])).abs().max())
         print(f"pipeline round {it}: max |cuda - reference| {err}")
@@ -90,8 +90,8 @@ def test_full_pipeline_replays_reference_golden(cuda_device):
     for it in range(rounds):
         tape = NoiseTape(s_pose, dev)
         for _ in range(it * (pn + 1) + 1):
-            tape.randn(B, 294, 1, 143)  # earlier rounds' draws and this round's x_T
-        noises = {i: tape.randn(B, 294, 1, 143) for i in range(pn - 1, -1, -1)}
+            tape.randn(B, 294, 1, T - 1)  # earlier rounds' draws and this round's x_T
+        noises = {i: tape.randn(B, 294, 1, T - 1) for i in range(pn - 1, -1, -1)}
         batch = {'cond': torch.from_numpy(g[f"r{it}_cond"]).to(dev)}
         for i, nxt in ((6, f"r{it}_xt5"), (1, f"r{it}_xt0"), (0, f"r{it}_val_pose")):
             dp._randn_like = lambda x, _n=noises[i]: _n

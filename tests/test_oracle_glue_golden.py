@@ -64,17 +64,17 @@ def test_projection_guidance_matches_reference_autograd():
 
 
 def test_pipeline_oracle_matches_reference_rounds():
-    """2 clips x 144 frames, 10-step TrajNet / 12-step guided PoseNet, 2 rounds (round 2 through TrajControl)."""
+    """2 clips x 32 frames, 10-step TrajNet / 12-step guided PoseNet, 2 rounds (round 2 through TrajControl)."""
     from rohm_b200.posenet import PoseNet
     from rohm_b200.trajnet import TrajNet
     g = golden("pipeline.npz")
-    B, tn, pn, rounds, s_in, s_pose, s_traj = [int(v) for v in g["meta"]]
+    B, tn, pn, rounds, s_in, s_pose, s_traj, frames = [int(v) for v in g["meta"]]
     ds_pose = synthetic.make_dataset('pose', seed=3, realistic_std=True)
     ds_traj = synthetic.make_dataset('traj', seed=3, realistic_std=True)
     sd_pose = synthetic.synth_state_dict(PoseNet(dataset=ds_pose, body_feat_dim=294, latent_dim=512, traj_feat_dim=22), 1)
     mk = lambda c: TrajNet(time_dim=32, mid_dim=512, cond_dim=13, traj_feat_dim=13, trajcontrol=c, repr_abs_only=True)
     sd_traj, sd_ctrl = synthetic.synth_state_dict(mk(False), 2), synthetic.synth_state_dict(mk(True), 4)
-    pose, traj = synthetic.pipeline_batches(B, s_in, ds_pose)
+    pose, traj = synthetic.pipeline_batches(B, s_in, ds_pose, frames=frames)
     res = pipeline_oracle.run_rounds(sd_pose, sd_traj, sd_ctrl, ds_pose, ds_traj, synthetic.smplx_like_model(0), pose, traj,
                                      1000, tn, rounds, NoiseTape(s_pose), NoiseTape(s_traj),
                                      pose_respacing=PIPELINE_POSE_RESPACING, teacher=g, teacher_steps=(6, 1, 0))

@@ -366,15 +366,17 @@ def gen_glue(ref):
 
 POSE_RESPACING = "12" + ",0" * 19
 POSE_RECORDED_STEPS = (6, 5, 1, 0)
+# Twelve [B, 294, 1, frames - 1] float32 states are stored: 32 frames keep the fixture under 1 MB.
+PIPELINE_FRAMES = 32
 
 
 def gen_pipeline(ref):
     """BASELINE config 4 in miniature, driven through the UNMODIFIED reference: the call sequence of
     test_amass_full.py:231-384 (TrajNet -> host glue -> PoseNet with in-loop skating guidance, 2 rounds, round 2 through
-    TrajControl) on 2 clips x 144 frames with 10-step TrajNet and 12-step PoseNet schedules (every PoseNet step guided)."""
+    TrajControl) on 2 clips x 32 frames with 10-step TrajNet and 12-step PoseNet schedules (every PoseNet step guided)."""
     get_repr_smplx = ref.mr.get_repr_smplx
     out = {}
-    B, Tn_steps, Pn_steps, rounds = 2, 10, 12, 2
+    B, Tn_steps, Pn_steps, rounds, frames = 2, 10, 12, 2, PIPELINE_FRAMES
     ds_pose = synthetic.make_dataset('pose', seed=3, realistic_std=True)
     ds_traj = synthetic.make_dataset('traj', seed=3, realistic_std=True)
     body = _StubBody()
@@ -391,7 +393,7 @@ def gen_pipeline(ref):
             timestep_respacing=POSE_RESPACING, device='cpu')
     dt = mk(args, gd=ref.gdt, return_class=ref.respace.SpacedDiffusionTrajNet, num_diffusion_timesteps=Tn_steps, device='cpu')
     dc = mk(args, gd=ref.gdt, return_class=ref.respace.SpacedDiffusionTrajNet, num_diffusion_timesteps=Tn_steps, device='cpu')
-    pose, traj = synthetic.pipeline_batches(B, 71, ds_pose)
+    pose, traj = synthetic.pipeline_batches(B, 71, ds_pose, frames=frames)
     tfd, pfd = ds_traj.traj_feat_dim, ds_traj.pose_feat_dim
     val_pose = None
     with _patched_th(ref.gdp, 72), _patched_th(ref.gdt, 73):
@@ -462,7 +464,7 @@ def gen_pipeline(ref):
             out[f"r{it}_cond"] = pose['cond'].detach().numpy()
             out[f"r{it}_val_pose"] = val_pose.detach().numpy()
             print(f"pipeline round {it}: |val_traj| {float(val_traj.abs().max()):.3f} |val_pose| {float(val_pose.abs().max()):.3f}")
-    out["meta"] = np.array([B, Tn_steps, Pn_steps, rounds, 71, 72, 73])
+    out["meta"] = np.array([B, Tn_steps, Pn_steps, rounds, 71, 72, 73, frames])
     np.savez_compressed(os.path.join(OUT, "pipeline.npz"), **out)
     print("pipeline.npz")
 
